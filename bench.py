@@ -25,6 +25,10 @@ FM IQ at 1.1025 MS/s per GPU (weak scaling).  A "step" is one pass of the chain 
               the neighbour's samples wait for them (lrb200_graph_execute_shard).  HALO = lrb200_graph_halo().
   check     : every rank re-computes windows of its output with the numpy oracle run cold from HALO samples before the
               window (the first window straddles the rank's left chunk boundary) and the run FAILS on a mismatch.
+  --dump-outputs DIR : after the timed steps, what the last one computed (the chain's audio output) goes to DIR/audio.npy
+              (float32; DIR/audio_rank<r>.npy per rank for N > 1).  Inputs are seeded, so two builds run with the same
+              arguments can be compared output for output.  Beyond DUMP_BYTES in all, a fixed, seeded sample of the outputs is
+              written instead, with the sampled output indices beside it (<name>_index.npy, float64).
   --impl reference : the C restatement of the reference's CPU path (oracle/lr_oracle.c: VOLK dot-product FIRs and the
               overlap-save FIRs the reference defaults to with FFTW; the faster one is timed) on all usable host
               cores -- the reference stack (LuaJIT/VOLK/liquid/FFTW) is not installable here.  Does not load the
@@ -44,6 +48,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # write nothing into the tree, which may be read-only (oracle/cbuild.py: the same for the native build)
 
 RATE = 1102500.0
 TUNE_OFFSET = -250e3
@@ -57,6 +62,7 @@ ALG_BYTES_FIR = 16.0                        # plain complex FIR: 8 in + 8 out
 ALG_BYTES_CFG2 = 8.0 + 8.0 / 5.0            # translator + FIR + /5 fused: 9.6 B per input sample
 FP32_PEAK_TFLOPS = 74.0                     # packed FFMA2, measured on this pool's B200 with tools/ubench.cu (DESIGN.md 3)
 WORKLOADS = {"wbfm_mono_256Mi": 268435450, "wbfm_mono_8Gi": 8589934575}
+DUMP_BYTES = 64 << 20                       # --dump-outputs: at most this many bytes in all
 METRIC = "WBFM-mono chain Msamples/s (input samples) @N B200; FIR-128 HBM GB/s vs roofline"
 CHAIN = "Tuner(-250e3,200e3,5)>FreqDiscriminator(1.25)>Lowpass(128,15e3)>FMDeemphasis(75e-6)>Downsampler(5)"
 TOLERANCE = ("1e-5*max(1,|ref|_inf) against the pinned oracle (north_star); the reference's own specs use 1e-6 absolute "
@@ -230,6 +236,24 @@ def _oracle_from(O, x, n0):
     return ch.process(x)
 
 
+def dump_outputs(out_dir, name, y, budget):
+    """Write the 1-D float array `y` (numpy, or a torch tensor on the device) to out_dir/<name>.npy.  When it exceeds `budget`
+    bytes, a sample of it is written instead: sorted output indices drawn with a fixed seed (the same set in every run with
+    the same arguments), stored as <name>_index.npy in float64 (exact for any index below 2**53)."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = int(y.shape[0])
+    if n * 4 > budget:
+        idx = np.unique(np.random.default_rng(0).integers(0, n, budget // 12))
+        np.save(os.path.join(out_dir, name + "_index.npy"), idx.astype(np.float64))
+        if not isinstance(y, np.ndarray):
+            import torch
+            idx = torch.from_numpy(idx).to(y.device)
+        y = y[idx]
+    if not isinstance(y, np.ndarray):
+        y = y.cpu().numpy()
+    np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(y, np.float32))
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -349,6 +373,8 @@ def run_b200(args):
     sampler.mark(t_host0, time.monotonic())
     ms_total = e0.elapsed_time(e1)
     launches = lib.lrb200_launch_count() - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, "audio" if world == 1 else "audio_rank%d" % rank, y[:int(n_out.value)], DUMP_BYTES // world)
     tt = torch.tensor([ms_total], device="cuda", dtype=torch.float64)
     if world > 1:
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -766,14 +792,16 @@ def run_reference(args):
         rates[name] = cpu_rate(olib, x, trial, taps, cores, fft, out, 0.5, 4)[0]
     best = max(rates, key=rates.get)
     fft = 1 if best == "overlap_save_fft" else 0
-    steps = max(1, args.steps)
+    steps = args.steps
     warm = max(3, args.warmup)
     for _ in range(warm):
         cpu_chain_call(olib, x, n, taps, cores, fft, out)
     t0 = time.perf_counter()
     for _ in range(steps):
-        cpu_chain_call(olib, x, n, taps, cores, fft, out)
+        n_out = cpu_chain_call(olib, x, n, taps, cores, fft, out)
     el = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, "audio", out[:n_out], DUMP_BYTES)
     v = n * steps / el / 1e6
     emit(json.dumps({
         "impl": "reference", "metric": METRIC,
@@ -819,7 +847,10 @@ def main():
     ap.add_argument("--no-check", action="store_true", help="skip the oracle window check of the run's output")
     ap.add_argument("--check", action="store_true", help="(default) compare output windows with the oracle and fail on mismatch")
     ap.add_argument("--profile", action="store_true", help="profiling run (ncu): skip the e2e, FIR-128 sweep and CPU legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

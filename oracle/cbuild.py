@@ -3,28 +3,32 @@ infrastructure only: imported by tests/, __graft_entry__ and bench.py, never by 
 import ctypes
 import os
 import subprocess
+import tempfile
 from ctypes import POINTER, c_double, c_float, c_int, c_long, c_uint32, c_uint64, c_void_p
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
-def build(native=False):
+def build(native=False, out_dir=HERE):
     target = "liblr_oracle_native.so" if native else "liblr_oracle.so"
-    path = os.path.join(HERE, target)
+    path = os.path.join(out_dir, target)
     src = os.path.join(HERE, "lr_oracle.c")
     if not os.path.exists(path) or os.path.getmtime(path) < os.path.getmtime(src):
-        subprocess.run(["make", "-C", HERE, target], check=True, capture_output=True)
+        subprocess.run(["make", "-C", HERE, "OUT=" + out_dir, path], check=True, capture_output=True)
     return path
 
 
 def load(native=False):
-    try:
-        path = build(native)
-    except Exception:
-        if not native:
-            raise
-        path = build(False)
-    lib = ctypes.CDLL(path)
+    """`native`: the -march=native build, compiled into a temporary directory (removed again once the library is loaded)
+    so that a timing run writes nothing into the source tree; the portable build if that compile fails."""
+    if native:
+        with tempfile.TemporaryDirectory(prefix="lr_oracle_") as d:
+            try:
+                lib = ctypes.CDLL(build(True, d))
+            except Exception:
+                lib = ctypes.CDLL(build(False))
+    else:
+        lib = ctypes.CDLL(build(False))
     lib.lro_wbfm_chain.restype = c_long
     lib.lro_wbfm_chain.argtypes = [c_void_p, c_long, c_uint64, c_void_p, c_int, c_int, c_double, c_float,
                                    c_void_p, c_int, c_void_p, c_void_p, c_int, c_void_p, c_int, c_long]

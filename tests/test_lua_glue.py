@@ -3,6 +3,7 @@ is executed under a test interpreter in tests/test_lua_exec.py); these tests mak
 and must be current, every lrb200_* symbol the Lua code calls must be declared (LuaJIT raises "missing declaration"
 otherwise), every helper / method it calls must be defined by the glue or be part of the reference's block API, and the
 block structure of every file must balance."""
+import json
 import os
 import re
 import subprocess
@@ -107,8 +108,8 @@ def test_lua_block_structure_balances():
             assert text.count(a) == text.count(b), "%s: unbalanced %s%s" % (f, a, b)
 
 
-# (reference file, field or method the glue relies on) -- verified against the reference tree when it is present (the build
-# container); on the GPU box /root/reference does not exist and the test is skipped
+# (reference file, field or method the glue relies on) -- each pair was found in the LuaRadio tree by
+# tests/golden/make_block_goldens.py (tests/golden/reference_hooks.json); a new one is checked there before it is listed
 GLUE_RELIES_ON = [
     ("radio/blocks/signal/frequencytranslator.lua", "self.offset"), ("radio/blocks/signal/frequencydiscriminator.lua", "self.gain"),
     ("radio/blocks/signal/downsampler.lua", "self.factor"), ("radio/blocks/signal/iirfilter.lua", "self.b_taps"),
@@ -140,21 +141,16 @@ GLUE_RELIES_ON = [
 
 
 def test_fields_and_hooks_the_glue_relies_on_exist_in_the_reference():
-    import pytest
-    ref = os.environ.get("LUARADIO_REFERENCE", "/root/reference")
-    if not os.path.isdir(ref):
-        pytest.skip("reference tree not present on this machine")
-    missing = []
-    for rel, needle in GLUE_RELIES_ON:
-        text = open(os.path.join(ref, rel)).read()
-        if needle not in text:
-            missing.append((rel, needle))
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_hooks.json")) as f:
+        hooks = json.load(f)
+    found = {tuple(p) for p in hooks["found"]}
+    missing = [p for p in GLUE_RELIES_ON if p not in found]
     assert not missing, missing
     # every class the glue patches is registered by the reference (radio/blocks/init.lua, radio/composites/init.lua)
-    reg = open(os.path.join(ref, "radio/blocks/init.lua")).read()
+    reg = set(hooks["registered_blocks"])
     glue = open(os.path.join(LUA, "blocks_patch.lua")).read() + open(os.path.join(LUA, "firfilter_patch.lua")).read()
     for cls in set(re.findall(r"radio\.(\w+Block|\w+Source|\w+Sink)\b", glue)) | set(re.findall(r"\b(\w+Block) = \"", glue)):
-        assert re.search(r"\b%s\b" % cls, reg), "%s is not a reference block" % cls
+        assert cls in reg, "%s is not a reference block" % cls
 
 
 def test_glue_parses_as_lua():

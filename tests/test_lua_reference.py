@@ -5,7 +5,10 @@ real block / composite files of the hot path are loaded from the reference tree 
 CompositeBlock:connect, and CompositeBlock:_prepare_to_run() runs for real: differentiate, crawl, pipes, rate validation,
 initialize, evaluation order.  The mock library logs what the glue asked of libluaradio_b200.
 
-This is the closest the build image gets to running the glue under LuaJIT; it skips where the reference tree is absent."""
+This is the closest a machine without LuaJIT gets to running the glue; those tests need the LuaRadio tree
+(tests/lua_reference_env.py: $LUARADIO_REFERENCE) and skip where it is absent.  The oracle pins at the end compare with
+what the reference's own blocks computed, stored under tests/golden/ (tests/golden/make_block_goldens.py), and run
+everywhere."""
 import numpy as np
 import pytest
 
@@ -16,7 +19,8 @@ import re
 from tests.lua_interp import LuaTable
 from tests.test_lua_exec import MockLib, read
 
-pytestmark = pytest.mark.skipif(not E.available(), reason="reference tree not present on this machine")
+needs_reference = pytest.mark.skipif(not E.available(), reason="LuaRadio tree not present (LUARADIO_REFERENCE)")
+GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 MOCK_ENDS = """
 local block = require('radio.core.block')
@@ -52,6 +56,7 @@ def taps_of(it, data, n):
     return np.array([it.f32._fstore[(id(it.f32.get_cell(data, i)), "value")] for i in range(n)], np.float64)
 
 
+@needs_reference
 def test_reference_classes_load_and_the_glue_patches_them(monkeypatch):
     it, lib, types = env(monkeypatch)
     radio = it.require("radio")
@@ -74,6 +79,7 @@ def test_reference_classes_load_and_the_glue_patches_them(monkeypatch):
     assert all(s.hash["process_func"] is b200.hash["process"] for s in de.hash["signatures"].array())
 
 
+@needs_reference
 def test_wbfm_mono_example_through_the_reference_prepare_to_run(monkeypatch):
     """examples/rtlsdr_wbfm_mono.lua:11-28 with a mock source and sink: after the reference's own _prepare_to_run() the seven
     concrete blocks are ONE GPUChainBlock, initialised from taps the reference's initialize() methods designed at the rates
@@ -139,6 +145,7 @@ def test_wbfm_mono_example_through_the_reference_prepare_to_run(monkeypatch):
     assert chain.hash["initialize"] is patch.hash["GPUChainBlock"].hash["initialize"]
 
 
+@needs_reference
 def test_composites_stereo_and_am_synchronous_through_the_reference(monkeypatch):
     """The reference's own WBFMStereoDemodulator and AMSynchronousDemodulator composites: their concrete blocks become one
     GPUDagBlock each, and the reference's rate validation and initialize pass over the members."""
@@ -180,6 +187,7 @@ def test_composites_stereo_and_am_synchronous_through_the_reference(monkeypatch)
     assert [c[0] for c in lib.calls].count("lrb200_dag_add_graph") >= 1
 
 
+@needs_reference
 def test_without_the_cuda_feature_the_reference_runs_untouched(monkeypatch):
     it, lib, types = env(monkeypatch)
     monkeypatch.setenv("LUARADIO_DISABLE_CUDA", "1")
@@ -199,6 +207,7 @@ def test_without_the_cuda_feature_the_reference_runs_untouched(monkeypatch):
     assert order == [3] and lib.calls == []
 
 
+@needs_reference
 def test_reference_run_loop_drives_the_chain(monkeypatch):
     """top:start() through the reference's own start() (forced single-process by the glue), _prepare_to_run() and the
     round-robin run loop (composite.lua:647-707, Block:run_once block.lua:493-556) with mock pipes: every source vector is
@@ -245,38 +254,24 @@ def test_reference_run_loop_drives_the_chain(monkeypatch):
     assert out_pipe.hash["queue"] == []
 
 
-def test_pll_oracle_pinned_against_the_reference_pll_lua_executed(monkeypatch):
-    """The reference ships no pll_spec, so the oracle's PLL used to be an unpinned restatement.  Here the reference's OWN
+def test_pll_oracle_pinned_against_the_reference_pll_lua_executed():
+    """The reference ships no pll_spec, so the oracle's PLL used to be an unpinned restatement.  The reference's OWN
     radio/blocks/signal/pll.lua (instantiate, initialize, the process() loop: VCO, phase detector, loop filter, clamp, wrap)
-    is executed statement by statement in the interpreter on float32-faithful sample cells (tests/lua_reference_env.py:
-    Float32Types) and compared with oracle/lr_oracle.py: PLL on a 19 kHz pilot in noise, in two calls (state carried),
-    through acquisition and lock."""
+    was executed statement by statement in the interpreter on float32-faithful sample cells (tests/lua_reference_env.py:
+    Float32Types; stored in tests/golden/blocks_ref_executed.npz) and is compared with oracle/lr_oracle.py: PLL on a 19 kHz
+    pilot in noise, in two calls (state carried), through acquisition and lock."""
     from oracle import lr_oracle as O
-    it, lib, types = env(monkeypatch)
-    monkeypatch.setenv("LUARADIO_DISABLE_CUDA", "1")           # the stock reference block, no glue
-    rate, n = 220500.0, 2400
-    rng = np.random.default_rng(7)
-    t = np.arange(2 * n)
-    x = (0.8 * np.exp(2j * np.pi * 19011.0 / rate * t + 0.4j) + 0.05 * (rng.standard_normal(2 * n) + 1j * rng.standard_normal(2 * n))).astype(np.complex64)
-    blk = it.run("""
-        local PLLBlock = require('radio.blocks.signal.pll')
-        local types = require('radio.types')
-        local blk = PLLBlock(100, 18950, 19050, 2)
-        blk:differentiate({types.ComplexFloat32})
-        blk.inputs[1].pipe = {get_rate = function () return 220500 end}
-        blk:initialize()
-        return blk
-    """)[0]
+    g = np.load(os.path.join(GOLDEN_DIR, "blocks_ref_executed.npz"))
+    rate = 220500.0
+    x = g["pll_x"]
     ref = O.PLL(100, 18950, 19050, 2, rate)
-    for part in (x[:n], x[n:]):
-        out, err = it.call(it.index(blk, "process"), [blk, it.f32.vector_from_numpy(part)])
-        got_out, got_err = it.f32.to_numpy(out), it.f32.to_numpy(err)
+    for part, got_out, got_err in zip(np.split(x, 2), np.split(g["pll_out"], 2), np.split(g["pll_err"], 2)):
         exp_out, exp_err = ref.process(part)
         assert np.max(np.abs(got_err - exp_err)) <= 1e-7 and np.max(np.abs(got_out - exp_out)) <= 1e-7
         assert np.array_equal(got_err, exp_err) and np.array_equal(got_out, exp_out)          # the same float32 cells, bit for bit
     # the loop did something: it pulled in from the band centre (19 000 Hz) towards the 19 011 Hz pilot and the error settled
     assert abs(float(np.mean(exp_err[-400:]))) < 0.05 and np.std(exp_err[:200]) > np.std(exp_err[-200:]) * 0.5
-    f_locked = blk.hash["freq_locked"] * rate / (2 * np.pi)
+    f_locked = float(g["pll_freq_locked"]) * rate / (2 * np.pi)
     assert 19000.5 < f_locked < 19030 and f_locked == pytest.approx(ref.freq * rate / (2 * np.pi), abs=1e-9)
 
 
@@ -314,18 +309,17 @@ REF_CHAIN = """
 """
 
 
-def test_oracle_chain_against_the_reference_chain_executed(monkeypatch):
-    """SURVEY 8c lists "no full WBFM chain vector" among the gaps the reference's golden vectors leave.  Here the stock
-    reference runs the whole examples/rtlsdr_wbfm_mono.lua chain itself: its pure-Lua process() branches (the ones it uses
-    without VOLK / liquid: frequencytranslator.lua:91-112, firfilter.lua:228-307, downsampler.lua:45-56,
-    frequencydiscriminator.lua:66-90, iirfilter.lua:111-181), its composites, its CompositeBlock run loop -- executed in the
-    test interpreter on float32-faithful sample cells, fed in three ragged vectors -- and the numpy oracle's chain is compared
-    with what the reference's sink received.  (The pure-Lua FIR accumulates in float32 cells, the oracle in float64: hence a
-    tolerance -- the reference specs' own 1e-6; the measured difference is 4.5e-8.)"""
+def test_oracle_chain_against_the_reference_chain_executed():
+    """SURVEY 8c lists "no full WBFM chain vector" among the gaps the reference's golden vectors leave.  The stock reference
+    ran the whole examples/rtlsdr_wbfm_mono.lua chain itself (tests/golden/make_chain_golden.py, REF_CHAIN above): its
+    pure-Lua process() branches (the ones it uses without VOLK / liquid: frequencytranslator.lua:91-112,
+    firfilter.lua:228-307, downsampler.lua:45-56, frequencydiscriminator.lua:66-90, iirfilter.lua:111-181), its composites,
+    its CompositeBlock run loop -- executed in the test interpreter on float32-faithful sample cells, fed in three ragged
+    vectors -- and the numpy oracle's chain is compared with what the reference's sink received
+    (tests/golden/wbfm_chain_ref_executed.npz).  (The pure-Lua FIR accumulates in float32 cells, the oracle in float64: hence
+    a tolerance -- the reference specs' own 1e-6; the measured difference is 4.5e-8.)"""
     from oracle import lr_oracle as O
-    monkeypatch.setenv("LUARADIO_DISABLE_CUDA", "1")
-    it, lib, types = env(monkeypatch)
-    monkeypatch.setenv("LUARADIO_DISABLE_CUDA", "1")
+    g = np.load(os.path.join(GOLDEN_DIR, "wbfm_chain_ref_executed.npz"))
     rate = 1102500.0
     n = 1650
     rng = np.random.default_rng(11)
@@ -333,15 +327,11 @@ def test_oracle_chain_against_the_reference_chain_executed(monkeypatch):
     audio = np.sin(2 * np.pi * 3000.0 / rate * t)
     x = (0.9 * np.exp(1j * (2 * np.pi * 250e3 / rate * t + 2 * np.pi * 75e3 / rate * np.cumsum(audio)))
          + 0.02 * (rng.standard_normal(n) + 1j * rng.standard_normal(n))).astype(np.complex64)
-    run = it.run(REF_CHAIN)[0]
-    from tests.lua_interp import to_lua
-    parts = [x[:700], x[700:701], x[701:]]
-    got = it.call(run, [to_lua([it.f32.vector_from_numpy(p) for p in parts])])[0]
-    y = np.concatenate([it.f32.to_numpy(v) for v in got.array()])
+    assert np.array_equal(x, g["x"]) and list(g["splits"]) == [0, 700, 701, n]
+    y = g["y"]
     ref = O.Chain(O.tuner(-250e3, 200e3, 5, rate), O.FrequencyDiscriminator(1.25), O.lowpass_filter(128, 15e3, rate / 5, False),
                   O.IIRFilter(*O.fm_deemphasis_taps(75e-6, rate / 5), False), O.Downsampler(5)).process(x)
     assert len(y) == len(ref) == n // 25
-    assert lib.calls == []                                               # the stock reference, no library behind it
     scale = max(1.0, float(np.max(np.abs(ref))))
     err = float(np.max(np.abs(y - ref)))
     print("reference-executed chain vs oracle: max |diff| = %.3g over %d outputs" % (err, len(y)))
@@ -349,6 +339,7 @@ def test_oracle_chain_against_the_reference_chain_executed(monkeypatch):
     assert np.max(np.abs(ref)) > 1e-3                                    # a live signal came out of the filters' transient
 
 
+@needs_reference
 def test_top_spec_topology_through_the_reference_run_loop(monkeypatch):
     """tests/top_spec.lua:14-55's shape: two sources into MultiplyConjugateBlock (two outside feeds: it stays a block of its
     own, HOST-pointer handle, process(x, y) -> lrb200_block_execute_multi), then Lowpass -> FrequencyDiscriminator ->
@@ -396,36 +387,24 @@ def test_top_spec_topology_through_the_reference_run_loop(monkeypatch):
     assert calls[-2:] == ["lrb200_graph_max_output", "lrb200_graph_flush"] and sink.hash["vectors"] == 3      # two vectors + the flushed tail
 
 
-def test_discriminator_first_sample_signed_zero_artefact(monkeypatch):
+def test_discriminator_first_sample_signed_zero_artefact():
     """frequencydiscriminator.lua:33,72: the first sample is multiplied by conj(ComplexFloat32()) and atan2f sees a product of
     signed zeros -- pi / gain when both parts of the first sample are negative, 0 in the three other quadrants.  The
-    reference's own pure-Lua process() executed on float32-faithful cells, the oracle, and (on the GPU) both the stand-alone
-    and the fused discriminator must agree on it (tests/test_gpu_stream.py::test_wbfm_mono_chain_reference_executed_golden*)."""
+    reference's own pure-Lua process() executed on float32-faithful cells (stored in tests/golden/blocks_ref_executed.npz),
+    the oracle, and (on the GPU) both the stand-alone and the fused discriminator must agree on it
+    (tests/test_gpu_stream.py::test_wbfm_mono_chain_reference_executed_golden*)."""
     from oracle import lr_oracle as O
-    monkeypatch.setenv("LUARADIO_DISABLE_CUDA", "1")
-    it, lib, types = env(monkeypatch)
-    monkeypatch.setenv("LUARADIO_DISABLE_CUDA", "1")
-    make = it.run("""
-        local Disc = require('radio.blocks.signal.frequencydiscriminator')
-        local types = require('radio.types')
-        return function ()
-            local blk = Disc(1.25)
-            blk:differentiate({types.ComplexFloat32})
-            blk:initialize()
-            return blk
-        end
-    """)[0]
+    g = np.load(os.path.join(GOLDEN_DIR, "blocks_ref_executed.npz"))
     gain = 2 * np.pi * 1.25
-    for re, im, first in ((0.3, 0.2, 0.0), (-0.3, 0.2, 0.0), (0.3, -0.2, 0.0), (-0.3, -0.2, np.pi / gain)):
-        x = np.array([complex(re, im), complex(0.1, 0.4), complex(-0.2, 0.1)], np.complex64)
-        blk = it.call(make, [])[0]
-        out = it.call(it.index(blk, "process"), [blk, it.f32.vector_from_numpy(x)])[0]
-        got = it.f32.to_numpy(out)
+    for (re, im, first), x, got in zip(((0.3, 0.2, 0.0), (-0.3, 0.2, 0.0), (0.3, -0.2, 0.0), (-0.3, -0.2, np.pi / gain)),
+                                       g["disc_x"], g["disc_y"]):
+        assert np.array_equal(x, np.array([complex(re, im), complex(0.1, 0.4), complex(-0.2, 0.1)], np.complex64))
         exp = O.FrequencyDiscriminator(1.25).process(x)
         assert np.max(np.abs(got - exp)) <= 3e-8, (re, im, got, exp)          # one float32 ulp in the gain scaling
         assert abs(float(got[0]) - first) <= 1e-7 and abs(float(exp[0]) - first) <= 1e-7, (re, im, got[0], exp[0])
 
 
+@needs_reference
 def test_entry_point_module(monkeypatch):
     """require('radio_b200')(radio): true with the backend active and the classes patched, false (and nothing touched) with the
     kill switch."""
