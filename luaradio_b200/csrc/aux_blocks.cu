@@ -378,6 +378,8 @@ struct PllBlock : Block {
         LRB_CHECK(cudaStreamSynchronize(ctx().stream));
         return 0;
     }
+    // the one block whose reset state is not zero (the loop starts at the middle of its frequency range), so d_state is
+    // not carried state: reset rewrites it here instead of zeroing it
     void reset_host() override { consumed = 0; set_state(ctx().stream); cudaStreamSynchronize(ctx().stream); }
     int run(const void*, size_t, void*, size_t*, cudaStream_t) override {
         set_error("pll has two outputs (out, error): use lrb200_block_execute_multi");
@@ -455,37 +457,24 @@ struct BinaryBlock : Block {
 
 struct DelayBlock : Block {
     long long D;
-    void* d_state[2] = {nullptr, nullptr};
-    int cur = 0;
+    Carried state;                  // last D inputs
     DelayBlock(unsigned num_samples, unsigned elem, bool dev) : D(num_samples) {
         name = "delay";
         in_size = out_size = elem;
         dev_ptrs = dev;
     }
-    ~DelayBlock() override { cudaFree(d_state[0]); cudaFree(d_state[1]); }
-    int init() override {
-        for (int i = 0; i < 2; ++i) {
-            LRB_CHECK(cudaMalloc(&d_state[i], (size_t)D * in_size));
-            LRB_CHECK(cudaMemset(d_state[i], 0, (size_t)D * in_size));
-        }
-        return 0;
-    }
-    void reset_host() override { consumed = 0; cur = 0; }
-    void state_buffers(std::vector<std::pair<void*, size_t>>& segs) override {
-        segs.push_back({d_state[0], (size_t)D * in_size});
-        segs.push_back({d_state[1], (size_t)D * in_size});
-    }
+    int init() override { return carry(state, (size_t)D * in_size); }
     long long memory_in() const override { return D; }
     int run(const void* dx, size_t n, void* dy, size_t* n_out, cudaStream_t s) override {
         *n_out = n;
         if (n == 0) return 0;
         const long long wpe = (long long)in_size / 4;
         const long long nw = (long long)n * wpe, Dw = D * wpe;
-        delay_kernel<<<ax_grid(nw > Dw ? nw : Dw), AX_THREADS, 0, s>>>((const uint32_t*)dx, (const uint32_t*)d_state[cur],
-                                                                        (uint32_t*)d_state[cur ^ 1], (uint32_t*)dy, nw, Dw);
+        delay_kernel<<<ax_grid(nw > Dw ? nw : Dw), AX_THREADS, 0, s>>>((const uint32_t*)dx, (const uint32_t*)state.in(),
+                                                                        (uint32_t*)state.out(), (uint32_t*)dy, nw, Dw);
         count_launch();
         LRB_CHECK(cudaGetLastError());
-        cur ^= 1;
+        state.flip();
         consumed += n;
         return 0;
     }
@@ -561,15 +550,6 @@ struct PsdBlock : Block {
 
 using namespace lrb;
 
-template <typename B>
-static lrb200_block_t* wrap_aux(B* b) {
-    if (!b) { set_error("out of memory"); return nullptr; }
-    if (b->init() != 0) { delete b; return nullptr; }
-    lrb200_block_t* h = new (std::nothrow) lrb200_block_s{b};
-    if (!h) { delete b; set_error("out of memory"); }
-    return h;
-}
-
 extern "C" {
 
 lrb200_block_t* lrb200_binary_create(const char* op, unsigned complex_data, unsigned flags) {
@@ -578,7 +558,7 @@ lrb200_block_t* lrb200_binary_create(const char* op, unsigned complex_data, unsi
     int code = o == "multiply" ? BIN_MUL : o == "multiplyconjugate" ? BIN_MULCONJ : o == "add" ? BIN_ADD : o == "subtract" ? BIN_SUB : -1;
     if (code < 0) { set_error("binary: unknown operation \"%s\" (multiply, multiplyconjugate, add, subtract)", o.c_str()); return nullptr; }
     if (code == BIN_MULCONJ && !complex_data) { set_error("binary: multiplyconjugate needs complex data"); return nullptr; }
-    return wrap_aux(new (std::nothrow) BinaryBlock(code, complex_data != 0, (flags & LRB200_DEVICE) != 0));
+    return wrap(make_block<BinaryBlock>(code, complex_data != 0, (flags & LRB200_DEVICE) != 0));
 }
 
 lrb200_block_t* lrb200_pll_create(double loop_bandwidth, double frequency_min, double frequency_max, double multiplier,
@@ -586,7 +566,7 @@ lrb200_block_t* lrb200_pll_create(double loop_bandwidth, double frequency_min, d
     if (ctx().device < 0 && lrb200_init(0) != 0) return nullptr;
     if (!(rate > 0.0) || !(loop_bandwidth > 0.0) || !std::isfinite(multiplier)) { set_error("pll: rate and loop bandwidth must be positive"); return nullptr; }
     if (!(frequency_min <= frequency_max)) { set_error("pll: frequency_min must not exceed frequency_max"); return nullptr; }
-    return wrap_aux(new (std::nothrow) PllBlock(loop_bandwidth, frequency_min, frequency_max, multiplier, rate, (flags & LRB200_DEVICE) != 0));
+    return wrap(make_block<PllBlock>(loop_bandwidth, frequency_min, frequency_max, multiplier, rate, (flags & LRB200_DEVICE) != 0));
 }
 
 int lrb200_pll_set_mode(lrb200_block_t* q, int mode) {
@@ -601,7 +581,7 @@ lrb200_block_t* lrb200_delay_create(unsigned num_samples, unsigned elem_size, un
     if (ctx().device < 0 && lrb200_init(0) != 0) return nullptr;
     if (num_samples == 0) { set_error("delay: number of samples must be greater than 0"); return nullptr; }
     if (elem_size != 4 && elem_size != 8) { set_error("delay: elem_size must be 4 or 8"); return nullptr; }
-    return wrap_aux(new (std::nothrow) DelayBlock(num_samples, elem_size, (flags & LRB200_DEVICE) != 0));
+    return wrap(make_block<DelayBlock>(num_samples, elem_size, (flags & LRB200_DEVICE) != 0));
 }
 
 lrb200_block_t* lrb200_psd_create(unsigned num_samples, const float32_t* window, double scale, unsigned logarithmic,
@@ -613,8 +593,8 @@ lrb200_block_t* lrb200_psd_create(unsigned num_samples, const float32_t* window,
     }
     if (!window) { set_error("psd: missing window"); return nullptr; }
     if (!(scale > 0.0)) { set_error("psd: scale (sample rate * window energy) must be positive"); return nullptr; }
-    return wrap_aux(new (std::nothrow) PsdBlock((int)num_samples, (const float*)window, scale, logarithmic != 0, complex_data != 0,
-                                                (flags & LRB200_DEVICE) != 0));
+    return wrap(make_block<PsdBlock>((int)num_samples, (const float*)window, scale, logarithmic != 0, complex_data != 0,
+                                     (flags & LRB200_DEVICE) != 0));
 }
 
 }  // extern "C"

@@ -61,9 +61,17 @@ static int ensure_init() {
 static constexpr size_t HOST_CHUNK = (size_t)1 << 24;   // samples per staged chunk in host mode
 
 Block::~Block() {
-    cudaFree(d_in);
-    cudaFree(d_out);
-    for (void* p : m_bufs) cudaFree(p);
+    for (void* p : staging) cudaFree(p);
+}
+
+int Block::carry(Carried& c, size_t bytes, int slots) {
+    for (int i = 0; i < slots; ++i) {
+        LRB_CHECK(cudaMalloc(&c.slot[i], bytes));
+        LRB_CHECK(cudaMemset(c.slot[i], 0, bytes));
+    }
+    c.bytes = bytes;
+    carried.push_back(&c);
+    return 0;
 }
 
 int Block::execute_multi(const void* const* x, int nin, size_t n, void* const* y, int nout, size_t* n_out) {
@@ -78,30 +86,30 @@ int Block::execute_multi(const void* const* x, int nin, size_t n, void* const* y
         if (n_out) *n_out = produced;
         return 0;
     }
-    if (m_bufs.empty()) { m_bufs.assign((size_t)(nin + nout), nullptr); m_caps.assign((size_t)(nin + nout), 0); }
+    if (staging.empty()) { staging.assign((size_t)(nin + nout), nullptr); staging_cap.assign((size_t)(nin + nout), 0); }
     size_t done = 0;
     std::vector<const void*> din((size_t)nin);
     std::vector<void*> dout((size_t)nout);
-    while (done < n || (n == 0 && done == 0)) {
+    while (done < n) {
         const size_t nc = n - done < HOST_CHUNK ? n - done : HOST_CHUNK;
         const size_t mo = max_output(nc);
         for (int i = 0; i < nin; ++i) {
-            if (reserve(&m_bufs[(size_t)i], &m_caps[(size_t)i], (nc ? nc : 1) * in_size) != 0) return -1;
-            if (nc) LRB_CHECK(cudaMemcpyAsync(m_bufs[(size_t)i], (const char*)x[i] + done * in_size, nc * in_size, cudaMemcpyHostToDevice, s));
-            din[(size_t)i] = m_bufs[(size_t)i];
+            if (reserve(&staging[(size_t)i], &staging_cap[(size_t)i], nc * in_size) != 0) return -1;
+            LRB_CHECK(cudaMemcpyAsync(staging[(size_t)i], (const char*)x[i] + done * in_size, nc * in_size, cudaMemcpyHostToDevice, s));
+            din[(size_t)i] = staging[(size_t)i];
         }
         for (int o = 0; o < nout; ++o) {
-            if (reserve(&m_bufs[(size_t)(nin + o)], &m_caps[(size_t)(nin + o)], (mo ? mo : 1) * out_size_of(o)) != 0) return -1;
-            dout[(size_t)o] = m_bufs[(size_t)(nin + o)];
+            if (reserve(&staging[(size_t)(nin + o)], &staging_cap[(size_t)(nin + o)], (mo ? mo : 1) * out_size_of(o)) != 0) return -1;
+            dout[(size_t)o] = staging[(size_t)(nin + o)];
         }
         size_t no = 0;
         if (run_multi(din.data(), nin, nc, dout.data(), nout, &no, s) != 0) return -1;
         for (int o = 0; o < nout; ++o)
             if (no) LRB_CHECK(cudaMemcpyAsync((char*)y[o] + produced * out_size_of(o), dout[(size_t)o], no * out_size_of(o), cudaMemcpyDeviceToHost, s));
+        // the staging buffers are reused by the next chunk: drain before overwriting them
         LRB_CHECK(cudaStreamSynchronize(s));
         produced += no;
         done += nc;
-        if (n == 0) break;
     }
     if (n_out) *n_out = produced;
     return 0;
@@ -125,45 +133,10 @@ int Block::reset() {
     return 0;
 }
 
-int Block::execute(const void* x, size_t n, void* y, size_t* n_out) {
-    cudaStream_t s = ctx().stream;
-    size_t produced = 0;
-    if (dev_ptrs) {
-        if (run(x, n, y, &produced, s) != 0) return -1;
-        if (n_out) *n_out = produced;
-        return 0;
-    }
-    size_t done = 0;
-    while (done < n) {
-        size_t nc = n - done < HOST_CHUNK ? n - done : HOST_CHUNK;
-        size_t mo = max_output(nc);
-        if (reserve(&d_in, &d_in_cap, nc * in_size) != 0) return -1;
-        if (reserve(&d_out, &d_out_cap, (mo ? mo : 1) * out_size) != 0) return -1;
-        LRB_CHECK(cudaMemcpyAsync(d_in, (const char*)x + done * in_size, nc * in_size, cudaMemcpyHostToDevice, s));
-        size_t no = 0;
-        if (run(d_in, nc, d_out, &no, s) != 0) return -1;
-        if (no) LRB_CHECK(cudaMemcpyAsync((char*)y + produced * out_size, d_out, no * out_size, cudaMemcpyDeviceToHost, s));
-        // the staging buffers are reused by the next chunk: drain before overwriting d_in
-        LRB_CHECK(cudaStreamSynchronize(s));
-        produced += no;
-        done += nc;
-    }
-    if (n_out) *n_out = produced;
-    return 0;
-}
-
-static inline void decim_plan(uint64_t consumed, unsigned D, size_t n, long long* first, long long* n_out) {
-    // downsampler.lua:45-53 in global-index form: outputs sit at global input index == 0 (mod D)
-    uint64_t r = consumed % D;
-    long long f = (long long)((D - r) % D);
-    *first = f;
-    *n_out = ((long long)n > f) ? (((long long)n - f + D - 1) / D) : 0;
-}
-
 // ---------------------------------------------------------------------------------------------
 // FIR (+ Hilbert)
 // ---------------------------------------------------------------------------------------------
-FirBlock::FirBlock(FirKind k, const void* taps_host, unsigned ntaps, unsigned decim, bool dev) {
+FirBlock::FirBlock(FirKind k, const void* taps_host, unsigned ntaps, unsigned decim, bool dev, bool rot, double turns_per_sample) {
     kind = k;
     M = (int)ntaps;
     D = (int)decim;
@@ -174,39 +147,29 @@ FirBlock::FirBlock(FirKind k, const void* taps_host, unsigned ntaps, unsigned de
     tap_size = (k == FIR_CCCF) ? 8 : 4;
     name = k == FIR_CRCF ? "fir_crcf" : k == FIR_CCCF ? "fir_cccf" : k == FIR_RRRF ? "fir_rrrf" : "hilbert";
     h_taps.assign((const char*)taps_host, (const char*)taps_host + (size_t)M * tap_size);
+    rotate = rot;
+    rot_turns = turns_per_sample;
+    rot_fix = turns_to_fix(turns_per_sample);
 }
 
 int FirBlock::init() {
     LRB_CHECK(cudaMalloc(&d_taps, (size_t)M * tap_size));
     LRB_CHECK(cudaMemcpy(d_taps, h_taps.data(), (size_t)M * tap_size, cudaMemcpyHostToDevice));
-    size_t hb = (size_t)(M > 1 ? M - 1 : 1) * in_size;
-    for (int i = 0; i < 2; ++i) {
-        LRB_CHECK(cudaMalloc(&d_hist[i], hb));
-        LRB_CHECK(cudaMemset(d_hist[i], 0, hb));
-    }
+    if (carry(hist, (size_t)(M > 1 ? M - 1 : 1) * in_size) != 0) return -1;
     return fast_init();
 }
 
 int FirBlock::set_pole(float c) {
-    for (int i = 0; i < 2; ++i) {
-        LRB_CHECK(cudaMalloc(&d_pole[i], sizeof(float)));
-        LRB_CHECK(cudaMemset(d_pole[i], 0, sizeof(float)));
-    }
+    if (carry(pole, sizeof(float)) != 0) return -1;
     has_pole = true;
     pole_c = c;
     return 0;
 }
 
 FirBlock::~FirBlock() {
-    cudaFree(d_pole[0]);
-    cudaFree(d_pole[1]);
     cudaFree(d_taps);
-    cudaFree(d_hist[0]);
-    cudaFree(d_hist[1]);
     fast_free();
 }
-
-size_t FirBlock::max_output(size_t n) const { return D == 1 ? n : n / D + 1; }
 
 static long long decay_samples(double c) {        // samples until |c|^k < 1e-12; < 0 if it never gets there
     const double a = std::fabs(c);
@@ -229,17 +192,8 @@ long long IirBlock::memory_in() const {
     return w < 0 ? -1 : w + nb;
 }
 
-void FirBlock::reset_host() { consumed = 0; cur = 0; pcur = 0; }
-void FirBlock::state_buffers(std::vector<std::pair<void*, size_t>>& segs) {
-    const size_t hb = (size_t)(M > 1 ? M - 1 : 1) * in_size;
-    segs.push_back({d_hist[0], hb});
-    segs.push_back({d_hist[1], hb});
-    if (has_pole) { segs.push_back({d_pole[0], sizeof(float)}); segs.push_back({d_pole[1], sizeof(float)}); }
-}
-
 int FirBlock::run(const void* dx, size_t n, void* dy, size_t* n_out, cudaStream_t s) {
-    long long first, no;
-    decim_plan(consumed, (unsigned)D, n, &first, &no);
+    const auto [first, no] = plan(n);
     *n_out = (size_t)no;
     if (n == 0) return 0;
     // the history for the next call depends only on x and the old history: side stream, concurrent with the filter
@@ -247,14 +201,14 @@ int FirBlock::run(const void* dx, size_t n, void* dy, size_t* n_out, cudaStream_
     cudaStream_t side = s;
     if (M > 1) {
         if (n >= SIDE_STREAM_MIN) side = side_fork(s);
-        if (launch_hist_update(dx, (long long)n, d_hist[cur], d_hist[cur ^ 1], M - 1, (int)in_size, side) != 0) return -1;
+        if (launch_hist_update(dx, (long long)n, hist.in(), hist.out(), M - 1, (int)in_size, side) != 0) return -1;
     }
     int rc = fast_run(dx, n, dy, first, no, s);
-    if (rc == 0) rc = launch_fir_generic(kind, dx, d_hist[cur], d_taps, M, D, first, no, dy, s) == 0 ? 1 : -1;
+    if (rc == 0) rc = launch_fir_generic(kind, dx, hist.in(), d_taps, M, D, first, no, dy, s) == 0 ? 1 : -1;
     side_join(s, side);
     if (rc < 0) return -1;
-    if (M > 1) cur ^= 1;
-    if (has_pole && no > 0) pcur ^= 1;
+    if (M > 1) hist.flip();
+    if (has_pole && no > 0) pole.flip();
     consumed += n;
     return 0;
 }
@@ -287,19 +241,11 @@ DiscrimBlock::DiscrimBlock(float gain_, bool dev) {
     dev_ptrs = dev;
     gain = gain_;
 }
-int DiscrimBlock::init() {
-    LRB_CHECK(cudaMalloc(&d_prev, sizeof(float2)));
-    LRB_CHECK(cudaMemset(d_prev, 0, sizeof(float2)));
-    return 0;
-}
-DiscrimBlock::~DiscrimBlock() { cudaFree(d_prev); }
-void DiscrimBlock::reset_host() { consumed = 0; }
-void DiscrimBlock::state_buffers(std::vector<std::pair<void*, size_t>>& segs) { segs.push_back({d_prev, sizeof(float2)}); }
 int DiscrimBlock::run(const void* dx, size_t n, void* dy, size_t* n_out, cudaStream_t s) {
     *n_out = n;
     if (n == 0) return 0;
-    if (launch_discrim((const float2*)dx, (const float2*)d_prev, (float*)dy, (long long)n, 1.0f / gain, s) != 0) return -1;
-    if (launch_copy_last(dx, (long long)n, d_prev, 8, s) != 0) return -1;
+    if (launch_discrim((const float2*)dx, (const float2*)prev.in(), (float*)dy, (long long)n, 1.0f / gain, s) != 0) return -1;
+    if (launch_copy_last(dx, (long long)n, prev.out(), 8, s) != 0) return -1;
     consumed += n;
     return 0;
 }
@@ -313,10 +259,8 @@ DownsampleBlock::DownsampleBlock(unsigned factor, unsigned elem, bool dev) {
     dev_ptrs = dev;
     D = (int)factor;
 }
-size_t DownsampleBlock::max_output(size_t n) const { return D == 1 ? n : n / D + 1; }
 int DownsampleBlock::run(const void* dx, size_t n, void* dy, size_t* n_out, cudaStream_t s) {
-    long long first, no;
-    decim_plan(consumed, (unsigned)D, n, &first, &no);
+    const auto [first, no] = plan(n);
     *n_out = (size_t)no;
     if (launch_downsample(dx, dy, first, no, D, (int)in_size, s) != 0) return -1;
     consumed += n;
@@ -337,39 +281,22 @@ IirBlock::IirBlock(bool cplx, const float* b_, unsigned nb_, const float* a_, un
     c = (na_ >= 2) ? (float)(-(double)a_[1] / a0) : 0.0f;
 }
 int IirBlock::init() {
-    size_t hb = (size_t)(nb > 1 ? nb - 1 : 1) * in_size;
-    for (int i = 0; i < 2; ++i) {
-        LRB_CHECK(cudaMalloc(&d_xhist[i], hb));
-        LRB_CHECK(cudaMemset(d_xhist[i], 0, hb));
-        LRB_CHECK(cudaMalloc(&d_ystate[i], in_size));
-        LRB_CHECK(cudaMemset(d_ystate[i], 0, in_size));
-    }
+    if (carry(xhist, (size_t)(nb > 1 ? nb - 1 : 1) * in_size) != 0 || carry(ystate, in_size) != 0) return -1;
     return iir_work_alloc(&work, (int)in_size);
 }
-IirBlock::~IirBlock() {
-    for (int i = 0; i < 2; ++i) { cudaFree(d_xhist[i]); cudaFree(d_ystate[i]); }
-    iir_work_free(&work);
-}
-size_t IirBlock::max_output(size_t n) const { return D == 1 ? n : n / D + 1; }
-void IirBlock::reset_host() { consumed = 0; cur = 0; }
-void IirBlock::state_buffers(std::vector<std::pair<void*, size_t>>& segs) {
-    const size_t hb = (size_t)(nb > 1 ? nb - 1 : 1) * in_size;
-    for (int i = 0; i < 2; ++i) { segs.push_back({d_xhist[i], hb}); segs.push_back({d_ystate[i], in_size}); }
-}
+IirBlock::~IirBlock() { iir_work_free(&work); }
 int IirBlock::run(const void* dx, size_t n, void* dy, size_t* n_out, cudaStream_t s) {
-    long long first_total, no_total;
-    decim_plan(consumed, (unsigned)D, n, &first_total, &no_total);
-    *n_out = (size_t)no_total;
+    *n_out = (size_t)plan(n).n_out;
     const long long maxn = iir_max_per_launch(work);
     size_t done = 0, produced = 0;
     while (done < n) {
         long long nc = (long long)(n - done) < maxn ? (long long)(n - done) : maxn;
-        long long first, no;
-        decim_plan(consumed, (unsigned)D, (size_t)nc, &first, &no);
+        const auto [first, no] = plan((size_t)nc);
         if (launch_iir1(complex_data, (const char*)dx + done * in_size, nc, (char*)dy + produced * out_size, b, nb, c,
-                        d_xhist[cur], d_xhist[cur ^ 1], d_ystate[cur], d_ystate[cur ^ 1], first, D, &work, s) != 0)
+                        xhist.in(), xhist.out(), ystate.in(), ystate.out(), first, D, &work, s) != 0)
             return -1;
-        cur ^= 1;
+        xhist.flip();
+        ystate.flip();
         consumed += (uint64_t)nc;
         done += (size_t)nc;
         produced += (size_t)no;
@@ -405,30 +332,16 @@ IirGeneralBlock::IirGeneralBlock(bool cplx, const float* b_, unsigned nb_, const
     }
     warm = (last + na + nb >= limit - 1) ? -1 : last + na + nb;
 }
-int IirGeneralBlock::init() {
-    for (int i = 0; i < 2; ++i) {
-        LRB_CHECK(cudaMalloc(&d_xhist[i], 10 * in_size));
-        LRB_CHECK(cudaMemset(d_xhist[i], 0, 10 * in_size));
-        LRB_CHECK(cudaMalloc(&d_yhist[i], 10 * in_size));
-        LRB_CHECK(cudaMemset(d_yhist[i], 0, 10 * in_size));
-    }
-    return 0;
-}
-IirGeneralBlock::~IirGeneralBlock() {
-    for (int i = 0; i < 2; ++i) { cudaFree(d_xhist[i]); cudaFree(d_yhist[i]); }
-}
-void IirGeneralBlock::reset_host() { consumed = 0; cur = 0; }
-void IirGeneralBlock::state_buffers(std::vector<std::pair<void*, size_t>>& segs) {
-    for (int i = 0; i < 2; ++i) { segs.push_back({d_xhist[i], 10 * in_size}); segs.push_back({d_yhist[i], 10 * in_size}); }
-}
+int IirGeneralBlock::init() { return carry(xhist, 10 * in_size) != 0 ? -1 : carry(yhist, 10 * in_size); }
 int IirGeneralBlock::run(const void* dx, size_t n, void* dy, size_t* n_out, cudaStream_t s) {
     *n_out = n;
     if (n == 0) return 0;
-    if (launch_iir_general(complex_data, dx, (long long)n, dy, b, nb, a, na, d_xhist[cur], d_yhist[cur], warm, s) != 0) return -1;
+    if (launch_iir_general(complex_data, dx, (long long)n, dy, b, nb, a, na, xhist.in(), yhist.in(), warm, s) != 0) return -1;
     // carried state: last nb-1 inputs of [xhist | x], last na-1 outputs of [yhist | y] (oldest first)
-    if (nb > 1 && launch_hist_update(dx, (long long)n, d_xhist[cur], d_xhist[cur ^ 1], nb - 1, (int)in_size, s) != 0) return -1;
-    if (na > 1 && launch_hist_update(dy, (long long)n, d_yhist[cur], d_yhist[cur ^ 1], na - 1, (int)in_size, s) != 0) return -1;
-    cur ^= 1;
+    if (nb > 1 && launch_hist_update(dx, (long long)n, xhist.in(), xhist.out(), nb - 1, (int)in_size, s) != 0) return -1;
+    if (na > 1 && launch_hist_update(dy, (long long)n, yhist.in(), yhist.out(), na - 1, (int)in_size, s) != 0) return -1;
+    xhist.flip();
+    yhist.flip();
     consumed += n;
     return 0;
 }
@@ -457,11 +370,8 @@ int C2fBlock::run(const void* dx, size_t n, void* dy, size_t* n_out, cudaStream_
 // =============================================================================================
 using namespace lrb;
 
-
-template <typename B>
-static lrb200_block_t* wrap(B* b) {
-    if (!b) { set_error("out of memory"); return nullptr; }
-    if (b->init() != 0) { delete b; return nullptr; }
+lrb200_block_t* lrb::wrap(Block* b) {
+    if (!b) return nullptr;
     lrb200_block_t* h = new (std::nothrow) lrb200_block_s{b};
     if (!h) { delete b; set_error("out of memory"); }
     return h;
@@ -638,7 +548,7 @@ static lrb200_block_t* fir_create(FirKind k, const void* taps, unsigned ntaps, u
     if (!taps || ntaps == 0) { set_error("fir: taps must be non-empty"); return nullptr; }
     if (decim == 0) { set_error("fir: decimation must be >= 1"); return nullptr; }
     if (k == FIR_HILBERT && (ntaps % 2) == 0) { set_error("hilbert: number of taps must be odd"); return nullptr; }
-    return wrap(new (std::nothrow) FirBlock(k, taps, ntaps, decim, (flags & LRB200_DEVICE) != 0));
+    return wrap(make_block<FirBlock>(k, taps, ntaps, decim, (flags & LRB200_DEVICE) != 0));
 }
 lrb200_fir_t* lrb200_fir_create_crcf(const float32_t* taps, unsigned ntaps, unsigned decim, unsigned flags) { return fir_create(FIR_CRCF, taps, ntaps, decim, flags); }
 lrb200_fir_t* lrb200_fir_create_cccf(const complex_float32_t* taps, unsigned ntaps, unsigned decim, unsigned flags) { return fir_create(FIR_CCCF, taps, ntaps, decim, flags); }
@@ -662,20 +572,20 @@ lrb200_hilbert_t* lrb200_hilbert_create(const float32_t* taps, unsigned ntaps, u
 lrb200_rotator_t* lrb200_rotator_create(double turns_per_sample, unsigned flags) {
     if (ensure_init() != 0) return nullptr;
     if (!std::isfinite(turns_per_sample)) { set_error("rotator: turns_per_sample is not finite"); return nullptr; }
-    return wrap(new (std::nothrow) RotatorBlock(turns_per_sample, (flags & LRB200_DEVICE) != 0));
+    return wrap(make_block<RotatorBlock>(turns_per_sample, (flags & LRB200_DEVICE) != 0));
 }
 
 lrb200_discrim_t* lrb200_discrim_create(float gain, unsigned flags) {
     if (ensure_init() != 0) return nullptr;
     if (!(gain != 0.0f) || !std::isfinite(gain)) { set_error("discrim: gain must be finite and non-zero"); return nullptr; }
-    return wrap(new (std::nothrow) DiscrimBlock(gain, (flags & LRB200_DEVICE) != 0));
+    return wrap(make_block<DiscrimBlock>(gain, (flags & LRB200_DEVICE) != 0));
 }
 
 lrb200_downsample_t* lrb200_downsample_create(unsigned factor, unsigned elem_size, unsigned flags) {
     if (ensure_init() != 0) return nullptr;
     if (factor == 0) { set_error("downsample: factor must be >= 1"); return nullptr; }
     if (elem_size != 4 && elem_size != 8) { set_error("downsample: elem_size must be 4 or 8"); return nullptr; }
-    return wrap(new (std::nothrow) DownsampleBlock(factor, elem_size, (flags & LRB200_DEVICE) != 0));
+    return wrap(make_block<DownsampleBlock>(factor, elem_size, (flags & LRB200_DEVICE) != 0));
 }
 
 static lrb200_block_t* iir_create(bool cplx, const float32_t* b, unsigned nb, const float32_t* a, unsigned na, unsigned flags) {
@@ -684,54 +594,49 @@ static lrb200_block_t* iir_create(bool cplx, const float32_t* b, unsigned nb, co
     if (nb > 10 || na > 10) { set_error("iir: at most 10 feed-forward and 10 feedback taps"); return nullptr; }
     if (a[0].value == 0.0f) { set_error("iir: a[0] must be non-zero"); return nullptr; }
     if (na > 2 || nb > 9)
-        return wrap(new (std::nothrow) IirGeneralBlock(cplx, (const float*)b, nb, (const float*)a, na, (flags & LRB200_DEVICE) != 0));
-    return wrap(new (std::nothrow) IirBlock(cplx, (const float*)b, nb, (const float*)a, na, (flags & LRB200_DEVICE) != 0));
+        return wrap(make_block<IirGeneralBlock>(cplx, (const float*)b, nb, (const float*)a, na, (flags & LRB200_DEVICE) != 0));
+    return wrap(make_block<IirBlock>(cplx, (const float*)b, nb, (const float*)a, na, (flags & LRB200_DEVICE) != 0));
 }
 lrb200_iir_t* lrb200_iir_create_rrrf(const float32_t* b, unsigned nb, const float32_t* a, unsigned na, unsigned flags) { return iir_create(false, b, nb, a, na, flags); }
 lrb200_iir_t* lrb200_iir_create_crcf(const float32_t* b, unsigned nb, const float32_t* a, unsigned na, unsigned flags) { return iir_create(true, b, nb, a, na, flags); }
 
 lrb200_block_t* lrb200_cmag_create(unsigned flags) {
     if (ensure_init() != 0) return nullptr;
-    return wrap(new (std::nothrow) C2fBlock(0, (flags & LRB200_DEVICE) != 0));
+    return wrap(make_block<C2fBlock>(0, (flags & LRB200_DEVICE) != 0));
 }
 lrb200_block_t* lrb200_c2r_create(unsigned flags) {
     if (ensure_init() != 0) return nullptr;
-    return wrap(new (std::nothrow) C2fBlock(1, (flags & LRB200_DEVICE) != 0));
+    return wrap(make_block<C2fBlock>(1, (flags & LRB200_DEVICE) != 0));
 }
 
 lrb200_block_t* lrb200_mulconst_create(float re, float im, unsigned complex_data, unsigned complex_constant, unsigned flags) {
     if (ensure_init() != 0) return nullptr;
     if (complex_constant && !complex_data) { set_error("mulconst: a complex constant needs complex data"); return nullptr; }
-    return wrap(new (std::nothrow) ScaleBlock(re, im, complex_data != 0, complex_constant != 0, (flags & LRB200_DEVICE) != 0));
+    return wrap(make_block<ScaleBlock>(re, im, complex_data != 0, complex_constant != 0, (flags & LRB200_DEVICE) != 0));
 }
 lrb200_block_t* lrb200_upsample_create(unsigned factor, unsigned elem_size, unsigned flags) {
     if (ensure_init() != 0) return nullptr;
     if (factor == 0) { set_error("upsample: factor must be >= 1"); return nullptr; }
     if (elem_size != 4 && elem_size != 8) { set_error("upsample: elem_size must be 4 or 8"); return nullptr; }
-    return wrap(new (std::nothrow) UpsampleBlock(factor, elem_size, (flags & LRB200_DEVICE) != 0));
+    return wrap(make_block<UpsampleBlock>(factor, elem_size, (flags & LRB200_DEVICE) != 0));
 }
 
 lrb200_block_t* lrb200_iqconv_create(const char* format, unsigned flags) {
     if (ensure_init() != 0) return nullptr;
-    Block* b = make_iqconv(format, (flags & LRB200_DEVICE) != 0);
-    if (!b) return nullptr;
-    return wrap(b);
+    return wrap(make_iqconv(format, (flags & LRB200_DEVICE) != 0));
 }
 
 lrb200_block_t* lrb200_realconv_create(const char* format, unsigned flags) {
     if (ensure_init() != 0) return nullptr;
-    Block* b = make_fileconv(format, false, 1, (flags & LRB200_DEVICE) != 0);
-    return b ? wrap(b) : nullptr;
+    return wrap(make_fileconv(format, false, 1, (flags & LRB200_DEVICE) != 0));
 }
 lrb200_block_t* lrb200_iqsink_create(const char* format, unsigned flags) {
     if (ensure_init() != 0) return nullptr;
-    Block* b = make_fileconv(format, true, 2, (flags & LRB200_DEVICE) != 0);
-    return b ? wrap(b) : nullptr;
+    return wrap(make_fileconv(format, true, 2, (flags & LRB200_DEVICE) != 0));
 }
 lrb200_block_t* lrb200_realsink_create(const char* format, unsigned flags) {
     if (ensure_init() != 0) return nullptr;
-    Block* b = make_fileconv(format, true, 1, (flags & LRB200_DEVICE) != 0);
-    return b ? wrap(b) : nullptr;
+    return wrap(make_fileconv(format, true, 1, (flags & LRB200_DEVICE) != 0));
 }
 
 // ---- synthetic sources -------------------------------------------------------------------------

@@ -638,15 +638,15 @@ int FirBlock::set_algorithm(int a) {
 
 int FirBlock::fast_run(const void* dx, size_t n, void* dy, long long first, long long n_out, cudaStream_t s) {
     if (poly && algo != LRB200_FIR_FFT && kind == FIR_RRRF)
-        return launch_polyphase_rrrf(poly, (const float*)dx, (const float*)d_hist[cur], (long long)n, (float*)dy, first, n_out, s,
-                                     pole_c, has_pole ? (const float*)d_pole[pcur] : nullptr, has_pole ? (float*)d_pole[pcur ^ 1] : nullptr);
+        return launch_polyphase_rrrf(poly, (const float*)dx, (const float*)hist.in(), (long long)n, (float*)dy, first, n_out, s,
+                                     pole_c, has_pole ? (const float*)pole.in() : nullptr, has_pole ? (float*)pole.out() : nullptr);
     if (has_pole) { set_error("fir: the fused output-rate pole needs the real polyphase kernel"); return -1; }
     if (poly && algo != LRB200_FIR_FFT)
-        return launch_polyphase_crcf(poly, (const float2*)dx, (const float2*)d_hist[cur], (long long)n, (float2*)dy,
+        return launch_polyphase_crcf(poly, (const float2*)dx, (const float2*)hist.in(), (long long)n, (float2*)dy,
                                      first, n_out, false, 0, consumed, s);
     const int eff = effective_algorithm();
     if (gen_poly && eff == LRB200_FIR_DIRECT) {
-        const int rc = launch_poly_generic(kind, dx, d_hist[cur], h_taps.data(), M, D, first, (long long)n, n_out, dy, s);
+        const int rc = launch_poly_generic(kind, dx, hist.in(), h_taps.data(), M, D, first, (long long)n, n_out, dy, s);
         if (rc != 0) return rc;
     }
     if (!fast || eff != LRB200_FIR_FFT) {
@@ -665,7 +665,7 @@ int FirBlock::fast_run(const void* dx, size_t n, void* dy, long long first, long
         const long long nb = ((long long)n + FD_HOP - 1) / FD_HOP;
         for (int p0 = 0; p0 < fast->nparts; p0 += FD_MAXPC) {
             FdlArgs a;
-            a.x = (const float2*)dx; a.hist = (const float2*)d_hist[cur]; a.y = (float2*)dy;
+            a.x = (const float2*)dx; a.hist = (const float2*)hist.in(); a.y = (float2*)dy;
             a.H = fast->d_H + (size_t)p0 * FF_N; a.tw = fast->d_tw; a.n = (long long)n;
             a.pc = std::min(FD_MAXPC, fast->nparts - p0);
             a.nblocks = nb;
@@ -686,7 +686,7 @@ int FirBlock::fast_run(const void* dx, size_t n, void* dy, long long first, long
         if (b_hi < b_lo) b_hi = b_lo;
         if (b_lo > nblocks) { b_lo = nblocks; b_hi = nblocks; }
         FftArgs a;
-        a.x = dx; a.hist = d_hist[cur]; a.y = dy; a.H = fast->d_H; a.tw = fast->d_tw; a.E = fast->d_E;
+        a.x = dx; a.hist = hist.in(); a.y = dy; a.H = fast->d_H; a.tw = fast->d_tw; a.E = fast->d_E;
         a.n = (long long)n; a.b_lo = b_lo; a.b_hi = b_hi; a.nwork = 0; a.first = first;
         a.turns_fix = rot_fix; a.g0 = consumed; a.M = Mp; a.D = D;
         // edge work list: blocks [0, b_lo) and [b_hi, nblocks); the kernel maps e -> (e < b_lo ? e : b_hi + e - b_lo)

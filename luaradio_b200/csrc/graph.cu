@@ -123,11 +123,11 @@ struct Graph {
                     }
                     if (used == 1 && fir_ok && f2->M <= 513) {
                         // translator folded into the overlap-save kernel (any taps, complex taps included)
-                        FirBlock* nf = new (std::nothrow) FirBlock(f2->kind, f2->h_taps.data(), (unsigned)f2->M, (unsigned)(d3 ? d3->D : 1), true);
-                        if (!nf) { set_error("out of memory"); return -1; }
-                        nf->set_rotation(rot->turns);      // (the fused translator forces the overlap-save path: algo is moot)
+                        // (the fused translator forces the overlap-save path: algo is moot)
+                        FirBlock* nf = make_block<FirBlock>(f2->kind, f2->h_taps.data(), (unsigned)f2->M, (unsigned)(d3 ? d3->D : 1), true,
+                                                            true, rot->turns);
+                        if (!nf) return -1;
                         nf->name = f2->kind == FIR_CCCF ? "rot+fir_cccf" : "rot+fir_crcf";
-                        if (nf->init() != 0) { delete nf; return -1; }
                         fused.push_back(nf); st = nf; used = d3 ? 3 : 2;
                     }
                 }
@@ -142,10 +142,9 @@ struct Graph {
                     if (up && f2 && f2->D == 1 && (f2->kind == FIR_CRCF || f2->kind == FIR_RRRF) && f2->in_size == up->out_size) {
                         DownsampleBlock* d3 = (j + 2 < blocks.size()) ? dynamic_cast<DownsampleBlock*>(blocks[j + 2]) : nullptr;
                         if (d3 && d3->in_size != f2->out_size) d3 = nullptr;
-                        InterpFirBlock* nb = new (std::nothrow) InterpFirBlock(f2->kind == FIR_CRCF, (const float*)f2->h_taps.data(), f2->M,
-                                                                               up->L, d3 ? d3->D : 1, sc != nullptr, sc ? sc->cre : 1.0f, true);
-                        if (!nb) { set_error("out of memory"); return -1; }
-                        if (nb->init() != 0) { delete nb; return -1; }
+                        InterpFirBlock* nb = make_block<InterpFirBlock>(f2->kind == FIR_CRCF, (const float*)f2->h_taps.data(), f2->M,
+                                                                        up->L, d3 ? d3->D : 1, sc != nullptr, sc ? sc->cre : 1.0f, true);
+                        if (!nb) return -1;
                         fused.push_back(nb); st = nb; used = (j - i) + 2 + (d3 ? 1 : 0);
                     }
                 }
@@ -178,10 +177,9 @@ struct Graph {
                                 if (t - k >= 0 && t - k < fir->M) acc += g[(size_t)k] * (double)h[t - k];
                             hc[(size_t)t] = (float)acc;
                         }
-                        FirBlock* nf = new (std::nothrow) FirBlock(FIR_RRRF, hc.data(), (unsigned)Mc, (unsigned)Dd, true);
-                        if (!nf) { set_error("out of memory"); return -1; }
+                        FirBlock* nf = make_block<FirBlock>(FIR_RRRF, hc.data(), (unsigned)Mc, (unsigned)Dd, true);
+                        if (!nf) return -1;
                         nf->set_algorithm(fir->algo);
-                        if (nf->init() != 0) { delete nf; return -1; }
                         if (nf->poly && nf->algo != LRB200_FIR_FFT && polyphase_pole_ok((float)cp)) {
                             // the pole's memory (|c^D|^64 <= 1e-8) fits the kernel's own warm-up: ONE stage
                             if (nf->set_pole((float)cp) != 0) { delete nf; return -1; }
@@ -191,9 +189,8 @@ struct Graph {
                             st = nf; used = 3;
                         } else if (nf->poly) {      // only worth it when the polyphase kernel has this shape
                             const float one = 1.0f, a2[2] = {1.0f, (float)(-cp)};     // cp == c^D
-                            IirBlock* ni = new (std::nothrow) IirBlock(false, &one, 1, a2, 2, true);
-                            if (!ni) { delete nf; set_error("out of memory"); return -1; }
-                            if (ni->init() != 0) { delete nf; delete ni; return -1; }
+                            IirBlock* ni = make_block<IirBlock>(false, &one, 1, a2, 2, true);
+                            if (!ni) { delete nf; return -1; }
                             nf->label = "fir*iir1_rrrf(" + std::to_string(Mc) + ",/" + std::to_string(Dd) + ")";
                             nf->name = nf->label.c_str();
                             ni->name = "pole_rrrf";
@@ -207,10 +204,9 @@ struct Graph {
                 if (used == 1 && fir && fir->D == 1 && fir->kind != FIR_HILBERT && i + 1 < blocks.size()) {
                     DownsampleBlock* d2 = dynamic_cast<DownsampleBlock*>(blocks[i + 1]);
                     if (d2 && d2->in_size == fir->out_size) {
-                        FirBlock* nf = new (std::nothrow) FirBlock(fir->kind, fir->h_taps.data(), (unsigned)fir->M, (unsigned)d2->D, true);
-                        if (!nf) { set_error("out of memory"); return -1; }
+                        FirBlock* nf = make_block<FirBlock>(fir->kind, fir->h_taps.data(), (unsigned)fir->M, (unsigned)d2->D, true);
+                        if (!nf) return -1;
                         nf->set_algorithm(fir->algo);      // FIRFilterBlock(taps, use_fft) survives the fusion
-                        if (nf->init() != 0) { delete nf; return -1; }
                         fused.push_back(nf); st = nf; used = 2;
                     }
                 }
@@ -218,10 +214,9 @@ struct Graph {
                     DownsampleBlock* d2 = dynamic_cast<DownsampleBlock*>(blocks[i + 1]);
                     if (d2 && d2->in_size == iir->out_size) {
                         float a[2] = {1.0f, -iir->c};
-                        IirBlock* ni = new (std::nothrow) IirBlock(iir->complex_data, iir->b, (unsigned)iir->nb, a, 2, true);
-                        if (!ni) { set_error("out of memory"); return -1; }
+                        IirBlock* ni = make_block<IirBlock>(iir->complex_data, iir->b, (unsigned)iir->nb, a, 2, true);
+                        if (!ni) return -1;
                         ni->D = d2->D;
-                        if (ni->init() != 0) { delete ni; return -1; }
                         fused.push_back(ni); st = ni; used = 2;
                     }
                 }

@@ -355,9 +355,7 @@ Block* make_iqconv(const char* format, bool dev) {
     if (!format) { set_error("iqconv: format is NULL"); return nullptr; }
     for (const FmtInfo& f : FORMATS)
         if (std::strcmp(f.name, format) == 0) {
-            Block* b = new (std::nothrow) IqConvBlock(f, dev);
-            if (!b) set_error("out of memory");
-            return b;
+            return make_block<IqConvBlock>(f, dev);
         }
     set_error("Unsupported format (\"%s\")", format);     // iqfile.lua:46
     return nullptr;
@@ -367,9 +365,7 @@ Block* make_fileconv(const char* format, bool to_file, int comps, bool dev) {
     if (!format) { set_error("fileconv: format is NULL"); return nullptr; }
     for (const FmtInfo& f : FORMATS)
         if (std::strcmp(f.name, format) == 0) {
-            Block* b = new (std::nothrow) FileConvBlock(f, to_file, comps, dev);
-            if (!b) set_error("out of memory");
-            return b;
+            return make_block<FileConvBlock>(f, to_file, comps, dev);
         }
     set_error("Unsupported format (\"%s\")", format);
     return nullptr;

@@ -415,8 +415,6 @@ InterpFirBlock::InterpFirBlock(bool cdata, const float* taps_host, int ntaps, in
 InterpFirBlock::~InterpFirBlock() {
     cudaFree(d_taps);
     cudaFree(d_taps_tp);
-    cudaFree(d_hist[0]);
-    cudaFree(d_hist[1]);
 }
 int InterpFirBlock::init() {
     LRB_CHECK(cudaMalloc(&d_taps, sizeof(float) * (size_t)M));
@@ -437,15 +435,7 @@ int InterpFirBlock::init() {
             if (Hn < g.Tt) Hn = g.Tt;
         }
     }
-    for (int i = 0; i < 2; ++i) {
-        LRB_CHECK(cudaMalloc(&d_hist[i], in_size * (size_t)Hn));
-        LRB_CHECK(cudaMemset(d_hist[i], 0, in_size * (size_t)Hn));
-    }
-    return 0;
-}
-void InterpFirBlock::state_buffers(std::vector<std::pair<void*, size_t>>& segs) {
-    segs.emplace_back(d_hist[0], in_size * (size_t)Hn);
-    segs.emplace_back(d_hist[1], in_size * (size_t)Hn);
+    return carry(hist, in_size * (size_t)Hn);
 }
 uint64_t InterpFirBlock::outputs_before(uint64_t idx) const { return (idx * (uint64_t)L + (uint64_t)D - 1) / (uint64_t)D; }
 size_t InterpFirBlock::max_output(size_t n) const { return (size_t)(((unsigned long long)n * L) / D + 2); }
@@ -472,8 +462,8 @@ int InterpFirBlock::run(const void* dx, size_t n, void* dy, size_t* n_out, cudaS
         }
         P.c = has_scale ? scale : 1.0f;
 #define LRB_RS(LL, DD) case (LL) * 32 + (DD): \
-            if (complex_data) launch_rs<float2, LL, DD>(P, dx, d_hist[cur], dy, g.smem, s); \
-            else launch_rs<float, LL, DD>(P, dx, d_hist[cur], dy, g.smem, s); \
+            if (complex_data) launch_rs<float2, LL, DD>(P, dx, hist.in(), dy, g.smem, s); \
+            else launch_rs<float, LL, DD>(P, dx, hist.in(), dy, g.smem, s); \
             break;
         switch (L * 32 + D) {
             LRB_RS(2, 1) LRB_RS(3, 1) LRB_RS(4, 1) LRB_RS(5, 1) LRB_RS(6, 1) LRB_RS(7, 1) LRB_RS(8, 1)
@@ -488,7 +478,7 @@ int InterpFirBlock::run(const void* dx, size_t n, void* dy, size_t* n_out, cudaS
         const long long ntiles = ((long long)n + IT_TILE - 1) / IT_TILE;
         const int g = (int)std::min<long long>(ntiles, (long long)ctx().sm_count * 8);
         const size_t smem = (((size_t)Tt * L * sizeof(float) + 15) & ~(size_t)15) + (size_t)(Tt + IT_TILE) * in_size;
-#define LRB_IT2(T, LL, S) interp_tiled_kernel<T, LL, S><<<g, IT_THREADS, smem, s>>>((const T*)dx, (const T*)d_hist[cur], (T*)dy, d_taps_tp, (long long)n, Hn, Tt, scale, D, (long long)consumed * L, m_lo)
+#define LRB_IT2(T, LL, S) interp_tiled_kernel<T, LL, S><<<g, IT_THREADS, smem, s>>>((const T*)dx, (const T*)hist.in(), (T*)dy, d_taps_tp, (long long)n, Hn, Tt, scale, D, (long long)consumed * L, m_lo)
 #define LRB_IT(LL) \
         if (complex_data) { if (has_scale) LRB_IT2(float2, LL, true); else LRB_IT2(float2, LL, false); } \
         else { if (has_scale) LRB_IT2(float, LL, true); else LRB_IT2(float, LL, false); }
@@ -507,15 +497,15 @@ int InterpFirBlock::run(const void* dx, size_t n, void* dy, size_t* n_out, cudaS
         LRB_CHECK(cudaGetLastError());
     } else if (no > 0) {
         const int g = grid_for(no);
-#define LRB_IF(T, S) interp_fir_kernel<T, S><<<g, 256, 0, s>>>((const T*)dx, (const T*)d_hist[cur], (T*)dy, d_taps, no, m_lo, (long long)consumed, Hn, L, D, M, scale)
+#define LRB_IF(T, S) interp_fir_kernel<T, S><<<g, 256, 0, s>>>((const T*)dx, (const T*)hist.in(), (T*)dy, d_taps, no, m_lo, (long long)consumed, Hn, L, D, M, scale)
         if (complex_data) { if (has_scale) LRB_IF(float2, true); else LRB_IF(float2, false); }
         else { if (has_scale) LRB_IF(float, true); else LRB_IF(float, false); }
 #undef LRB_IF
         count_launch();
         LRB_CHECK(cudaGetLastError());
     }
-    if (launch_hist_update(dx, (long long)n, d_hist[cur], d_hist[cur ^ 1], Hn, (int)in_size, s) != 0) return -1;
-    cur ^= 1;
+    if (launch_hist_update(dx, (long long)n, hist.in(), hist.out(), Hn, (int)in_size, s) != 0) return -1;
+    hist.flip();
     consumed += n;
     return 0;
 }

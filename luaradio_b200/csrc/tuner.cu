@@ -658,17 +658,20 @@ int launch_polyphase_crcf(const PolyTaps* p, const float2* x, const float2* hist
 // ---------------------------------------------------------------------------------------------
 // TunerBlock: Rotator -> FIR(crcf) -> Downsampler as one stage of the graph
 // ---------------------------------------------------------------------------------------------
-struct TunerBlock : Block {
-    int M, D;
+struct TunerBlock : DecimatingBlock {
+    int M;
+    double turns;
+    std::vector<float> h_taps;
     PolyTaps* pt = nullptr;
-    void* d_hist[2] = {nullptr, nullptr};
-    void* d_prev[2] = {nullptr, nullptr};      // fused discriminator: previous tuner output (ping-pong)
-    int cur = 0, pcur = 0;
+    Carried hist;
+    Carried prev;                              // fused discriminator: previous tuner output
     bool disc = false;
     float gain = 1.f;
     std::string label;
 
-    TunerBlock(PolyTaps* p, float disc_gain) : M(p->M), D(p->D), pt(p) {
+    TunerBlock(double turns_per_sample, const float* taps, int ntaps, int decim, float disc_gain)
+        : M(ntaps), turns(turns_per_sample), h_taps(taps, taps + ntaps) {
+        D = decim;
         disc = disc_gain != 0.0f;
         gain = disc_gain;
         in_size = 8;
@@ -677,35 +680,18 @@ struct TunerBlock : Block {
         label = std::string(disc ? "tuner+discrim(" : "tuner(") + std::to_string(M) + ",/" + std::to_string(D) + ")";
         name = label.c_str();
     }
-    ~TunerBlock() override {
-        polyphase_release(pt);
-        for (int i = 0; i < 2; ++i) { cudaFree(d_hist[i]); cudaFree(d_prev[i]); }
-    }
+    ~TunerBlock() override { polyphase_release(pt); }
     int init() override {
-        size_t hb = (size_t)(M > 1 ? M - 1 : 1) * 8;
-        for (int i = 0; i < 2; ++i) {
-            LRB_CHECK(cudaMalloc(&d_hist[i], hb));
-            LRB_CHECK(cudaMemset(d_hist[i], 0, hb));
-            LRB_CHECK(cudaMalloc(&d_prev[i], 8));
-            LRB_CHECK(cudaMemset(d_prev[i], 0, 8));
-        }
-        return 0;
+        pt = polyphase_prepare(h_taps.data(), M, D, turns, true);
+        if (!pt) return -1;      // unsupported shape: the graph keeps the blocks separate
+        if (carry(hist, (size_t)(M > 1 ? M - 1 : 1) * 8) != 0) return -1;
+        return carry(prev, 8);
     }
-    size_t max_output(size_t n) const override { return n / D + 1; }
-    uint64_t outputs_before(uint64_t idx) const override { return (idx + D - 1) / D; }
     long long memory_in() const override { return M - 1 + (disc ? D : 0); }
     bool supports_lead_wait() const override { return true; }
     bool state_only_on_side_stream() const override { return true; }
-    void rate(unsigned* up, unsigned* down) const override { *up = 1; *down = (unsigned)D; }
-    void reset_host() override { consumed = 0; cur = pcur = 0; }
-    void state_buffers(std::vector<std::pair<void*, size_t>>& segs) override {
-        const size_t hb = (size_t)(M > 1 ? M - 1 : 1) * 8;
-        for (int i = 0; i < 2; ++i) { segs.push_back({d_hist[i], hb}); segs.push_back({d_prev[i], 8}); }
-    }
     int run(const void* dx, size_t n, void* dy, size_t* n_out, cudaStream_t s) override {
-        uint64_t r = consumed % (uint64_t)D;
-        long long first = (long long)(((uint64_t)D - r) % (uint64_t)D);
-        long long no = ((long long)n > first) ? (((long long)n - first + D - 1) / D) : 0;
+        const auto [first, no] = plan(n);
         *n_out = (size_t)no;
         if (n == 0) return 0;
         // the history for the next call depends only on x and the old history: update it on the side stream,
@@ -713,27 +699,22 @@ struct TunerBlock : Block {
         cudaStream_t side = s;
         if (M > 1) {
             if (n >= SIDE_STREAM_MIN) side = side_fork(s);
-            if (launch_hist_update(dx, (long long)n, d_hist[cur], d_hist[cur ^ 1], M - 1, 8, side) != 0) return -1;
+            if (launch_hist_update(dx, (long long)n, hist.in(), hist.out(), M - 1, 8, side) != 0) return -1;
         }
-        int rc = launch_polyphase_any(pt, (const float2*)dx, (const float2*)d_hist[cur], (long long)n, dy, first, no, true,
-                                      disc, consumed, (const float2*)d_prev[pcur], (float2*)d_prev[pcur ^ 1],
+        int rc = launch_polyphase_any(pt, (const float2*)dx, (const float2*)hist.in(), (long long)n, dy, first, no, true,
+                                      disc, consumed, (const float2*)prev.in(), (float2*)prev.out(),
                                       disc ? 1.0f / gain : 0.f, s);
         side_join(s, side);
         if (rc <= 0) { if (rc == 0) set_error("tuner: unsupported shape"); return -1; }
-        if (disc && no > 0) pcur ^= 1;
-        if (M > 1) cur ^= 1;
+        if (disc && no > 0) prev.flip();
+        if (M > 1) hist.flip();
         consumed += n;
         return 0;
     }
 };
 
 Block* make_tuner(double turns_per_sample, const float* taps, int ntaps, int decim, float disc_gain) {
-    PolyTaps* p = polyphase_prepare(taps, ntaps, decim, turns_per_sample, true);
-    if (!p) return nullptr;      // unsupported shape: the graph keeps the blocks separate
-    TunerBlock* t = new (std::nothrow) TunerBlock(p, disc_gain);
-    if (!t) { polyphase_release(p); set_error("out of memory"); return nullptr; }
-    if (t->init() != 0) { delete t; return nullptr; }
-    return t;
+    return make_block<TunerBlock>(turns_per_sample, taps, ntaps, decim, disc_gain);
 }
 
 }  // namespace lrb
